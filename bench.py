@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 3   # the reference algorithm on host cores
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W               # N>1: one rank per GPU, weak scaling
+    python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR   # also writes the last timed step's outputs
 
 A "step" = one full pass of the hot path over one batch: every one of the R replicas per GPU is simulated from
 t = 0 to end_time (reset -> arrival pre-pass -> list merge -> event loop -> on-device summary reduction
@@ -193,15 +194,13 @@ def _py_worker(args):
 
 
 def python_reference_leg(sc, cores):
-    """The reference's own Python loop, unmodified, timed here — only where its tree exists (/root/reference in the
-    build container, or baseline/_ref/); the GPU box has neither and the leg is skipped there."""
+    """The reference's own Python loop, unmodified, timed here — only when DCSIM_REFERENCE_ROOT names a checkout of
+    it; otherwise the leg is skipped."""
+    root = os.environ.get("DCSIM_REFERENCE_ROOT")
+    if not root or not os.path.isdir(os.path.join(root, "simcore")):
+        return None
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import ref_harness
-    root = next((p for p in (ref_harness.REFERENCE_ROOT, os.path.join(ROOT, "baseline", "_ref"))
-                 if os.path.isdir(os.path.join(p, "simcore"))), None)
-    if root is None:
-        return None
-    os.environ["DCSIM_REFERENCE_ROOT"] = root
     ref_harness.REFERENCE_ROOT = root
     import multiprocessing as mp
     import oracle_lib
@@ -278,6 +277,25 @@ def run_reference_arm(args, world, rank):
 
 
 # ---------------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, summary, first_replica, aggregate, sample_seed=0):
+    """Writes what one step hands its caller, so that two builds run with the same arguments can be compared file for
+    file: summary.npy (float64 [rows, SUMMARY_K], one row per replica), replica_ids.npy (the global id of each row)
+    and aggregate.npy (the all-reduced AGG_K-vector).  When every row does not fit in DUMP_BYTES, the rows are a
+    fixed, seeded sample in replica order."""
+    row_bytes = (summary.shape[1] + 1) * 8
+    cap = (DUMP_BYTES - aggregate.nbytes - 3 * 4096) // row_bytes          # 4096: room for each file's .npy header
+    rows = np.arange(len(summary))
+    if len(rows) > cap:
+        rows = np.sort(np.random.default_rng(sample_seed).choice(len(rows), cap, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "summary.npy"), np.ascontiguousarray(summary[rows], dtype=np.float64))
+    np.save(os.path.join(out_dir, "replica_ids.npy"), (first_replica + rows).astype(np.float64))
+    np.save(os.path.join(out_dir, "aggregate.npy"), np.asarray(aggregate, dtype=np.float64))
+
+
 def timed_batch(torch, dist, eng, stream, world, seed, first, warm=1):
     """`warm` untimed batches, then one batch timed with CUDA events on the launching stream; returns
     (ms max over ranks, pre-pass ms, event-loop ms) of this rank's timed batch."""
@@ -387,6 +405,8 @@ def run_b200(args, world, rank, local_rank):
     t1.record(stream)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.summary(), first, agg[args.warmup + args.steps - 1].cpu().numpy())
     elapsed_ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
     kernel_ms = [a.elapsed_time(b) for a, b in zip(k0, k1)]
     prepass_ms = sum(a.elapsed_time(b) for a, b in zip(p0, k0)) / args.steps
@@ -528,7 +548,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="tuning runs only: skip the end-to-end leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the side records (other BASELINE configs, strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/*.npy (rank 0, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm only")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
