@@ -148,6 +148,9 @@ struct dcsim {
 };
 
 static thread_local char g_create_err[512] = "";
+#ifdef DCSIM_DEVICE_TEST_HOOKS
+static double g_test_time_quantum = 0.0; /* TEST-ONLY builds: dcsim_test_set_time_quantum */
+#endif
 
 static int set_err(dcsim_t* h, int code, const char* fmt, const char* a = "", long long b = 0) {
   char* dst = h ? h->err : g_create_err;
@@ -453,6 +456,11 @@ static void fill_kparams(const dcsim_t* h, dcsim_kparams_t* P, uint64_t max_even
   P->ml_t = h->d_ml_t; P->ml_aux = h->d_ml_aux; P->ml_meta = h->d_ml_meta;
   P->arr_hdr = h->d_arr_hdr; P->cap_arr = h->cap_arr;
   P->max_transfer = h->max_transfer;
+#ifdef DCSIM_DEVICE_TEST_HOOKS
+  /* a rounded-up xfer_done instant may lie up to one quantum past t + transfer_s: the merge window must reach that far */
+  P->test_time_quantum = g_test_time_quantum;
+  P->max_transfer += g_test_time_quantum;
+#endif
   P->lat_hist = h->d_hist;
   P->mt_state = h->d_mt;
 }
@@ -685,6 +693,13 @@ int dcsim_launch_info(dcsim_t* h, dcsim_launch_info_t* out) {
 }
 
 const char* dcsim_last_error(const dcsim_t* h) { return h ? h->err : g_create_err; }
+
+#ifdef DCSIM_DEVICE_TEST_HOOKS
+/* TEST-ONLY (builds made with -DDCSIM_DEVICE_TEST_HOOKS, never the product library): every launch from now on rounds
+ * arrival and xfer_done instants up to a multiple of `q` (0 = off), like the oracle's and the host build's hook, so that
+ * same-instant events are common on the device too. */
+void dcsim_test_set_time_quantum(double q) { g_test_time_quantum = q; }
+#endif
 
 void dcsim_destroy(dcsim_t* h) {
   if (!h) return;

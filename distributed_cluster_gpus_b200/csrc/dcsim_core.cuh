@@ -471,6 +471,9 @@ struct dcsim_kparams_t {
   uint32_t _pad33;
   double end_eps;       /* end_time + 1e-9, the _schedule cut-off (SIM:161) */
   double max_transfer;  /* largest finite transfer_s[ingress][dc][jtype] of the scenario */
+#ifdef DCSIM_DEVICE_TEST_HOOKS
+  double test_time_quantum; /* TEST-ONLY device builds: see dcsim_test_quantize */
+#endif
 };
 
 /* ---- small typed views ------------------------------------------------------------------------ */
@@ -486,6 +489,7 @@ struct dcsim_ctx_t {
   dcsim_hdr_t* H;
   int lane;
   bool is_traced, is_logged;
+  bool is_ghost;          /* a lane group without a replica (dcsim_replica_step): reads, never writes */
   /* Hot scalars kept in registers and written back to the header when the launch ends.  seq: lane 0's copy is
    * authoritative (only lane 0 runs handlers); the others are warp-uniform. */
   uint32_t seq;          /* successful pushes (SIM:163) */
@@ -830,13 +834,20 @@ DCSIM_DEV double dcsim_size_from_raw(const dcsim_spec_t& sp, double raw, int jt)
   return v > sp.lognorm_floor ? v : sp.lognorm_floor;
 }
 
-/* TEST HOOK, host build only (see oracle/dcsim_oracle.c g_test_time_quantum): rounds arrival and xfer_done instants up
- * to a multiple of a quantum so that same-instant events become common and the tie-breaking below is exercised. */
-#ifdef DCSIM_HOST_EMU
-static double dcsim_test_time_quantum = 0.0;
-static inline double dcsim_test_quantize(double t) {
-  return (dcsim_test_time_quantum > 0.0 && !(t == DCSIM_INF)) ? ceil(t / dcsim_test_time_quantum) * dcsim_test_time_quantum : t;
+/* TEST HOOK (see oracle/dcsim_oracle.c g_test_time_quantum): rounds arrival and xfer_done instants up to a multiple of a
+ * quantum so that same-instant events become common and the tie-breaking below is exercised.  Compiled into the host
+ * build and into the test-only device builds made with -DDCSIM_DEVICE_TEST_HOOKS (tests/test_gpu_ties.py), where the
+ * quantum travels in the launch parameters (every caller has them as `P`); the product library has neither. */
+#if defined(DCSIM_HOST_EMU) || defined(DCSIM_DEVICE_TEST_HOOKS)
+DCSIM_DEV double dcsim_test_quantize_by(double q, double t) {
+  return (q > 0.0 && !(t == DCSIM_INF)) ? ceil(t / q) * q : t;
 }
+#endif
+#if defined(DCSIM_HOST_EMU)
+static double dcsim_test_time_quantum = 0.0;
+#define dcsim_test_quantize(t) dcsim_test_quantize_by(dcsim_test_time_quantum, (t))
+#elif defined(DCSIM_DEVICE_TEST_HOOKS)
+#define dcsim_test_quantize(t) dcsim_test_quantize_by(P->test_time_quantum, (t))
 #else
 #define dcsim_test_quantize(t) (t)
 #endif
@@ -1197,9 +1208,14 @@ DCSIM_DEV uint32_t* dcsim_list_seq_slot(dcsim_ctx_t& c, uint32_t m) {
  * The list's slot of the event set is never written: it stays +inf and takes part in (1) harmlessly.
  * Returns the winning candidate slot, -1 if all are +inf. */
 struct dcsim_omin_t { uint32_t hi, lo, seq; int slot; bool fresh; }; /* (1); fresh: just reduced, not yet in the header */
-/* Lane 0, after the event's first sync (every lane has read the header's copy by then): publishes a fresh (1). */
+/* Lane 0, after the event's first sync (every lane has read the header's copy by then): publishes a fresh (1).  Never
+ * from a ghost lane group: with nothing staged its `blk` IS replica n-1's block in HBM, and nothing orders its store
+ * against that replica's handler — landing after the handler had dirtied the event set again, it cleared cand_dirty over
+ * a stale minimum and replica n-1 popped events out of order (8 lanes, DCSIM_MODE_INPLACE: tests/test_gpu_launch_modes.py).
+ * A switched-off replica still publishes: its event set no longer changes, and a cache left dirty would make the whole
+ * warp re-reduce on every event until its last replica ends. */
 DCSIM_DEV void dcsim_omin_publish(dcsim_ctx_t& c, const dcsim_omin_t& o) {
-  if (o.fresh && c.lane == 0) {
+  if (o.fresh && c.lane == 0 && !c.is_ghost) {
     c.H->omin_t = dcsim_hilo_f64(o.hi, o.lo); c.H->omin_seq = o.seq; c.H->omin_slot = (uint32_t)o.slot; c.H->cand_dirty = 0u;
   }
 }
@@ -2166,6 +2182,7 @@ DCSIM_DEV uint32_t dcsim_replica_step(const dcsim_kparams_t* P, uint64_t r, char
   c.r = (uint32_t)r; /* n_replicas < 2^32 (checked by dcsim_create) */
   c.is_traced = !ghost && ((int64_t)r == P->rec.trace_replica);
   c.is_logged = !ghost && ((int64_t)r == P->rec.log_replica);
+  c.is_ghost = ghost;
   if (ghost) { /* a lane group without a replica (the batch's last warp): reads whatever is there, writes nothing */
     c.seq = 0u; c.now = 0.0; c.cursor = 0u;
     return dcsim_replica_run<CAP, RECG>(c, false);

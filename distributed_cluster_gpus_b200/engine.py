@@ -240,7 +240,10 @@ _CACHED_LOGGED = {"key": None, "engine": None}   # the one-replica companion eng
 
 
 def _cache_key(sp, n_replicas, device, cuda_stream):
-    return (sp.to_bytes(), int(n_replicas), int(device), int(cuda_stream), os.environ.get("DCSIM_RECORDS", ""))
+    # the launch geometry is fixed when the handle is created: an engine sized under other DCSIM_GROUP / DCSIM_RECORDS
+    # settings is not the engine the caller asked for
+    return (sp.to_bytes(), int(n_replicas), int(device), int(cuda_stream), os.environ.get("DCSIM_RECORDS", ""),
+            os.environ.get("DCSIM_GROUP", ""))
 
 
 def _drop_parked_batch_engine():
