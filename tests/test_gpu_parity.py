@@ -15,7 +15,7 @@ pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not has_cuda(), reason="needs 
 
 RTOL = 1e-9
 COUNT_COLS = (S.S_STATUS, S.S_EVENTS, S.S_JOBS_FINISHED, S.S_JOBS_CREATED, S.S_FIN_INF, S.S_FIN_TRN, S.S_RNG_WORDS,
-              S.S_SEQ, S.S_EV_ARRIVAL, S.S_EV_XFER, S.S_EV_FINISH, S.S_EV_LOG, S.S_DONE)
+              S.S_SEQ, S.S_EV_ARRIVAL, S.S_EV_XFER, S.S_EV_FINISH, S.S_EV_LOG, S.S_DONE, S.S_MAX_RUN, S.S_MAX_Q)
 FLOAT_COLS = (S.S_TOTAL_ENERGY_J, S.S_LAT_SUM, S.S_LAT_SUM_INF, S.S_LAT_SUM_TRN, S.S_LAST_T)
 DEVICE_SUPPORTED = golden_names()
 
